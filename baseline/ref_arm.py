@@ -135,24 +135,31 @@ def import_reference(num_devices: int = 1):
 
 
 # ------------------------------------------------------------------------------------------- headline workload
-def make_dataset(num_clients: int, batch: int, data_root: str, shape=(3, 32, 32), classes: int = 10, train_sizes=None):
+def synthetic_arrays(num_clients: int, batch: int, shape=(3, 32, 32), classes: int = 10, train_sizes=None, seed: int = 1):
+    """Class-conditional Gaussian images, ``2*batch`` train / ``batch`` test per client (or ``train_sizes[u]`` train):
+    the ``(train ids, train, test ids, test)`` tuple a ``generate_datasets`` returns.  Needs nothing but numpy, so
+    tests can rebuild the exact arrays the reference was given."""
     import numpy as np
+    rng = np.random.default_rng(seed)
+    means = rng.standard_normal((classes,) + tuple(shape)).astype(np.float32)
+    ids = list(range(num_clients))
+    train, test = {}, {}
+    for u in ids:
+        for store, n in ((train, train_sizes[u] if train_sizes else 2 * batch), (test, batch)):
+            y = rng.integers(0, classes, n)
+            x = (means[y] + rng.standard_normal((n,) + tuple(shape))).astype(np.float32)
+            store[u] = {"x": x, "y": y.astype(np.int64)}
+    return ids, train, ids, test
+
+
+def make_dataset(num_clients: int, batch: int, data_root: str, shape=(3, 32, 32), classes: int = 10, train_sizes=None):
     from blades.datasets.basedataset import BaseDataset
 
     class SyntheticCIFAR10(BaseDataset):
-        """CIFAR-10-shaped class-conditional Gaussian images, ``2*batch`` train / ``batch`` test per client."""
+        """CIFAR-10-shaped class-conditional Gaussian images (``synthetic_arrays``)."""
 
         def generate_datasets(self, path="./data", iid=True, alpha=0.1, num_clients=20, seed=1):
-            rng = np.random.default_rng(seed)
-            means = rng.standard_normal((classes,) + shape).astype(np.float32)
-            ids = list(range(num_clients))
-            train, test = {}, {}
-            for u in ids:
-                for store, n in ((train, train_sizes[u] if train_sizes else 2 * batch), (test, batch)):
-                    y = rng.integers(0, classes, n)
-                    x = (means[y] + rng.standard_normal((n,) + shape)).astype(np.float32)
-                    store[u] = {"x": x, "y": y.astype(np.int64)}
-            return ids, train, ids, test
+            return synthetic_arrays(num_clients, batch, shape, classes, train_sizes, seed)
 
     os.makedirs(data_root, exist_ok=True)
     return SyntheticCIFAR10(data_root=data_root, train_bs=batch, num_clients=num_clients, seed=1)

@@ -102,6 +102,19 @@ def build_model(name: str, classes: int):
             "resnet50": lambda: resnet50(num_classes=classes)}[name]()
 
 
+def dump_outputs(directory: str, arrays: dict, max_elems: int = 1 << 22) -> None:
+    """``<directory>/<name>.npy`` in float32 for every tensor of ``arrays``.  A tensor longer than ``max_elems`` is
+    stored as the same fixed, seeded sample of its coordinates in every run (at most 16 MB per array), so two builds
+    can be compared output for output."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().reshape(-1).float().cpu().numpy()
+        if a.size > max_elems:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, max_elems, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_ours(args) -> dict:
     import torch
 
@@ -160,6 +173,15 @@ def run_ours(args) -> dict:
     launches = _loader.LAUNCHES - launches0
     clocks = sampler.stop() if world.rank == 0 else {}
     eng.prestaged = None
+    if args.dump_outputs and world.rank == 0:
+        # what the last timed round handed back: the new global model, the aggregate the server applied and the
+        # per-client losses (rank 0's clients), parameters in the model's named_parameters() order
+        outs = {"theta": eng.gflat.to_reference_order(eng.gflat.theta)}
+        if sim.last_aggregate is not None and sim.last_aggregate.numel() == eng.d:
+            outs["aggregate"] = eng.gflat.to_reference_order(sim.last_aggregate.reshape(-1))
+        if eng.last_client_losses is not None:
+            outs["client_losses"] = eng.last_client_losses
+        dump_outputs(args.dump_outputs, outs)
 
     # ---------------- end-to-end through the public API ----------------
     h2d = d2h = 0
@@ -338,7 +360,12 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-port", action="store_true", help="skip the GPU-port comparison rounds (vs_baseline stays null)")
     ap.add_argument("--max-batched", type=int, default=0, help="clients per fused training pass (0 = all local)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed round computed to DIR/<name>.npy (float32, <= 64 MB in all); "
+                         "--impl ours only")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     if args.impl == "reference":
         if int(os.environ.get("RANK", "0")) == 0:

@@ -1,5 +1,5 @@
 #!/bin/bash
-# Final multi-GPU check: fault-injection (dead rank -> barrier timeout), sharded-vs-single cases, headline bench.
+# Final multi-GPU check: sharded-vs-single cases, headline bench.
 set -x
 N=${1:-2}
 mkdir -p gpurun_out

@@ -253,8 +253,11 @@ def test_channels_last_flat_layout_and_server():
         srv.apply_update(u)
     for p1, p2 in zip(m1.parameters(), m2.parameters()):
         assert torch.allclose(p1, p2, atol=1e-6)
-    x = torch.randn(8, 3, 32, 32)
-    assert torch.allclose(m1(x), m2(x), atol=1e-3)
+    x = torch.randn(8, 3, 32, 32).double()
+    # the parameter check above is the real comparison; this forward re-checks that both layouts hold the same model.
+    # In float64, because at these logit magnitudes (~200) the float32 CPU convolutions of the two memory formats round
+    # differently by more than the tolerance on some CPUs
+    assert torch.allclose(m1.double()(x), m2.double()(x), atol=1e-3)
 
 
 def test_batched_evaluation_equals_per_client_loop(tmp_path):

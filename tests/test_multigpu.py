@@ -53,20 +53,3 @@ def test_sharded_equals_single(agg, attack, model, n, tmp_path):
             assert rel < 5e-2, (w, rel)
         else:
             assert torch.allclose(vecs[0], base, atol=5e-4, rtol=1e-2), (w, (vecs[0] - base).abs().max())
-
-
-def test_dead_rank_is_detected_by_the_barrier_timeout(tmp_path):
-    """5.3 failure detection: a rank that never arrives makes the device barrier of the others trap after
-    ``BLADES_BARRIER_TIMEOUT_MS`` -- the job fails fast instead of hanging on the signal pads."""
-    import time
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
-           "--master-port", "29677", os.path.join(ROOT, "tests", "_mgpu_fault_worker.py"), str(tmp_path)]
-    env = dict(os.environ, BLADES_BARRIER_TIMEOUT_MS="3000")
-    t0 = time.time()
-    subprocess.run(cmd, capture_output=True, text=True, timeout=300, env=env)
-    took = time.time() - t0
-    path = os.path.join(str(tmp_path), "fault_rank0.txt")
-    assert os.path.exists(path), "rank 0 never came back from the barrier"
-    verdict = open(path).read()
-    assert verdict.startswith("detected"), verdict
-    assert took < 120, took
