@@ -220,8 +220,11 @@ class ByzantineClient(BladesClient):
     and/or ``omniscient_callback`` (reference client.py:231-253).
 
     ``fused_spec()`` is the B200 addition: an attacker may describe itself as a
-    coordinate-wise closed form (ALIE, IPM) so the aggregation kernel can insert
-    it as *virtual rows* instead of materialising f identical rows (SURVEY 7.2.3).
+    coordinate-wise closed form so the aggregation kernel can insert it as
+    *virtual rows* instead of materialising f identical rows (SURVEY 7.2.3):
+    ``{"kind": "alie" | "ipm", "param": p}``, or ``{"kind": "minmax" | "minsum", "param": 0.0,
+    "dev_type": "unit_vec" | "std" | "sign", "gamma_init": g0, "tol": t}`` (the scale of the
+    Min-Max / Min-Sum row is searched on the device, attackers/_agr.py).
     """
     _is_byzantine = True
 

@@ -3,7 +3,11 @@
 //    Box-Muller written straight into the client's row of the update matrix.
 //  * alie_ipm_row: standalone ALIE/IPM row (mean - z*std / -eps*mean over the honest rows) for
 //    aggregators that need the malicious row materialised (Gram-based ones); coordinate-wise
-//    aggregators use the fused prologue in coord_select.cu instead.
+//    aggregators use the fused prologue in coord_select.cu instead.  Kind 3 is the sign form mean - p*sign(mean)
+//    of the Min-Max / Min-Sum attacks; p may be read from device memory (param_ptr), where the scale solver of
+//    gram_solve.cu left it.
+//  * agr_deviation: the deviation vector q of Min-Max / Min-Sum over the honest rows (mean, std or sign(mean)),
+//    the extra row of the Gram pass whose result the scale solver searches.
 #include "common.cuh"
 
 __device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t (&k)[2]) {
@@ -47,12 +51,15 @@ extern "C" int bl_fill_normal(float* out, long long n, float mean, float stdv,
 struct AttackRowParams {
     const float* rows[BL_MAX_ROWS];   // honest rows
     int n_stat;
-    int kind;                         // 1 ALIE, 2 IPM
+    int kind;                         // 1 ALIE, 2 IPM, 3 sign (mean - param * sign(mean))
     float param;
     long long c0, c1;
     float* out[BL_MAX_ROWS];          // destination rows (the Byzantine clients' rows, local GPU)
     int n_out;
+    const float* param_ptr;           // non-null: the parameter is read from device memory instead of `param`
 };
+
+__device__ __forceinline__ float bl_signf(float x) { return (float)((x > 0.f) - (x < 0.f)); }
 
 __global__ void __launch_bounds__(256)
 attack_row_kernel(const __grid_constant__ AttackRowParams p) {
@@ -61,12 +68,15 @@ attack_row_kernel(const __grid_constant__ AttackRowParams p) {
     float s = 0.f;
     for (int i = 0; i < p.n_stat; ++i) s += bl_sanitize(bl_ldg_stream(p.rows[i] + c));
     const float mu = s / (float)p.n_stat;
+    const float param = p.param_ptr ? __ldg(p.param_ptr) : p.param;
     float m;
     if (p.kind == 1) {
         float q = 0.f;     // second pass hits L2 (the tile was just read)
         for (int i = 0; i < p.n_stat; ++i) { float d = bl_sanitize(__ldg(p.rows[i] + c)) - mu; q = fmaf(d, d, q); }
-        m = mu - p.param * sqrtf(q / (float)(p.n_stat - 1));
-    } else m = -p.param * mu;
+        m = mu - param * sqrtf(q / (float)(p.n_stat - 1));
+    } else if (p.kind == 3) {
+        m = mu - param * bl_signf(mu);
+    } else m = -param * mu;
     for (int j = 0; j < p.n_out; ++j) p.out[j][c] = m;
 }
 
@@ -77,3 +87,42 @@ extern "C" int bl_attack_rows(const AttackRowParams* p, void* stream) {
     return (int)cudaGetLastError();
 }
 extern "C" int bl_sizeof_attack_params() { return (int)sizeof(AttackRowParams); }
+
+// q[c] for c in [c0, c1): the deviation vector of Min-Max / Min-Sum over the honest rows, with the statistics of
+// attack_row_kernel (sanitised values, fp32 mean, two-pass unbiased std).  Under coordinate sharding every rank fills
+// only its own range (rows of peers are read over NVLink like the select kernels do); the Gram pass reads no more.
+struct DeviationParams {
+    const float* rows[BL_MAX_ROWS];   // honest rows
+    int n_stat;
+    int dev_type;                     // 0 mean, 1 std (unbiased), 2 sign(mean)
+    long long c0, c1;
+    float* q;                         // indexed by coordinate
+};
+
+__global__ void __launch_bounds__(256)
+agr_deviation_kernel(const __grid_constant__ DeviationParams p) {
+    const long long c = p.c0 + (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= p.c1) return;
+    float s = 0.f;
+    for (int i = 0; i < p.n_stat; ++i) s += bl_sanitize(bl_ldg_stream(p.rows[i] + c));
+    const float mu = s / (float)p.n_stat;
+    float q;
+    if (p.dev_type == 1) {
+        float v = 0.f;
+        for (int i = 0; i < p.n_stat; ++i) { float d = bl_sanitize(__ldg(p.rows[i] + c)) - mu; v = fmaf(d, d, v); }
+        q = sqrtf(v / (float)(p.n_stat - 1));
+    } else if (p.dev_type == 2) {
+        q = bl_signf(mu);
+    } else q = mu;
+    p.q[c] = q;
+}
+
+extern "C" int bl_agr_deviation(const DeviationParams* p, void* stream) {
+    if (p->n_stat < 1 || p->n_stat > BL_MAX_ROWS || p->dev_type < 0 || p->dev_type > 2) return -1;
+    if (p->dev_type == 1 && p->n_stat < 2) return -1;
+    const long long cols = p->c1 - p->c0;
+    if (cols <= 0) return 0;
+    agr_deviation_kernel<<<(unsigned)((cols + 255) / 256), 256, 0, (cudaStream_t)stream>>>(*p);
+    return (int)cudaGetLastError();
+}
+extern "C" int bl_sizeof_deviation_params() { return (int)sizeof(DeviationParams); }

@@ -13,6 +13,7 @@ struct SelectLargeParams {
     int mode, trim_b;
     long long c0, c1;
     BlEpilogue ep;
+    const float* virt_param_ptr;   // non-null: the virtual row's parameter is read from device memory
 };
 
 template <int NP>
@@ -35,12 +36,15 @@ coord_select_large_kernel(const __grid_constant__ SelectLargeParams p) {
             float s = 0.f;
             for (int i = 0; i < p.n_stat; ++i) s += tile[i * 33 + lane];
             const float mu = s / (float)p.n_stat;
+            const float param = bl_virt_param(p);
             float m;
             if (p.virt_kind == 1) {
                 float q = 0.f;
                 for (int i = 0; i < p.n_stat; ++i) { float d = tile[i * 33 + lane] - mu; q += d * d; }
-                m = mu - p.virt_param * sqrtf(q / (float)(p.n_stat - 1));
-            } else m = -p.virt_param * mu;
+                m = mu - param * sqrtf(q / (float)(p.n_stat - 1));
+            } else if (p.virt_kind == 3) {
+                m = mu - param * bl_sign(mu);
+            } else m = -param * mu;
             for (int i = n; i < N; ++i) tile[i * 33 + lane] = live ? m : INFINITY;
         }
         __syncthreads();

@@ -53,13 +53,18 @@ struct SelectParams {
     int n_real;               // number of real rows (<= NP)
     int n_stat;               // first n_stat rows enter the attack statistics
     int n_virtual;            // multiplicity f of the virtual row
-    int virt_kind;            // 0 none, 1 ALIE (mean - p*std_unbiased), 2 IPM (-p*mean)
+    int virt_kind;            // 0 none, 1 ALIE (mean - p*std_unbiased), 2 IPM (-p*mean), 3 sign (mean - p*sign(mean))
     float virt_param;
     int mode;                 // 0 trimmed mean, 1 median
     int trim_b;
     long long c0, c1;         // coordinate range owned by this launch
     BlEpilogue ep;
+    const float* virt_param_ptr;   // non-null: p is read from device memory (Min-Max / Min-Sum scale solver)
 };
+
+// the virtual row's parameter: the launch's constant, or the value a solver left in device memory
+template <class P>
+__device__ __forceinline__ float bl_virt_param(const P& p) { return p.virt_param_ptr ? __ldg(p.virt_param_ptr) : p.virt_param; }
 
 // Pipe balance (ncu: the ALU pipe -- FMNMX/ISETP/SEL, 16 lanes/clk/SMSP -- is the limiter): the sorting
 // network has to live on the ALU pipe, so everything else is written as FFMA / FADD.SAT arithmetic for
@@ -102,6 +107,7 @@ coord_select_kernel(const __grid_constant__ SelectParams p) {
 #pragma unroll
         for (int i = 0; i < NP; ++i) s = fmaf(v[i], __saturatef(fstat - (float)i), s);     // mask = [i < n_stat]
         const float mu = s / fstat;
+        const float param = bl_virt_param(p);
         if (p.virt_kind == 1) {
             float q = 0.f;
 #pragma unroll
@@ -109,9 +115,11 @@ coord_select_kernel(const __grid_constant__ SelectParams p) {
                 const float d = (v[i] - mu) * __saturatef(fstat - (float)i);
                 q = fmaf(d, d, q);
             }
-            m = mu - p.virt_param * sqrtf(q / (fstat - 1.f));
+            m = mu - param * sqrtf(q / (fstat - 1.f));
+        } else if (p.virt_kind == 3) {
+            m = mu - param * bl_sign(mu);
         } else {
-            m = -p.virt_param * mu;
+            m = -param * mu;
         }
     }
     // padding slots sort to the top: FLT_MAX (finite, so 0-weight products stay 0); n > NP - 8 by dispatch,
@@ -192,8 +200,8 @@ coord_select_part_kernel(const __grid_constant__ SelectParams p) {
     }
     const int f = p.n_virtual;
     float m = 0.f;
-    if (f > 0) m = p.n_stat == NP ? bl_virtual_value_all<NP>(a, b, total, p.virt_kind, p.virt_param)
-                                  : bl_virtual_value<NP>(a, b, p.n_stat, p.virt_kind, p.virt_param);
+    if (f > 0) m = p.n_stat == NP ? bl_virtual_value_all<NP>(a, b, total, p.virt_kind, bl_virt_param(p))
+                                  : bl_virtual_value<NP>(a, b, p.n_stat, p.virt_kind, bl_virt_param(p));
     bl_epilogue_store(p.ep, c, bl_trimmed_partition<NP, MIX, kSelectRollHalves>(a, b, m, f));
 }
 
@@ -257,8 +265,8 @@ coord_select_part_stage_kernel(const __grid_constant__ SelectParams p) {
             total = bl_total<NP>(a, b);
         }
         float m = 0.f;
-        if (f > 0) m = p.n_stat == NP ? bl_virtual_value_all<NP>(a, b, total, p.virt_kind, p.virt_param)
-                                      : bl_virtual_value<NP>(a, b, p.n_stat, p.virt_kind, p.virt_param);
+        if (f > 0) m = p.n_stat == NP ? bl_virtual_value_all<NP>(a, b, total, p.virt_kind, bl_virt_param(p))
+                                      : bl_virtual_value<NP>(a, b, p.n_stat, p.virt_kind, bl_virt_param(p));
         bl_epilogue_store(p.ep, p.c0 + t * kStageTile + tid, bl_trimmed_partition<NP, MIX>(a, b, m, f));
     }
 }
@@ -282,10 +290,11 @@ static bool select_partition_enabled() {
 }
 
 // The partition-only kernel applies when the real rows fill the padded size exactly, the trim count is a quarter of
-// them and a virtual row (if any) has multiplicity >= the trim count (select_part_core.cuh).
+// them and a virtual row (if any) has multiplicity >= the trim count (select_part_core.cuh).  Its virtual value needs
+// n_stat >= 2 only for the ALIE form (kind 1: the unbiased std); IPM (2) and sign (3) need the mean alone.
 static bool partition_applies(const SelectParams& p, int NP) {
     return p.mode == 0 && p.n_real == NP && p.trim_b * 4 == NP && (p.n_virtual == 0 || p.n_virtual >= p.trim_b)
-           && (p.n_virtual == 0 || p.n_stat >= 2 || p.virt_kind != 1) && select_partition_enabled();
+           && (p.n_virtual == 0 || p.n_stat >= 2 || p.virt_kind == 2 || p.virt_kind == 3) && select_partition_enabled();
 }
 
 // Compare-exchange mix (see bl_ce): BLADES_SELECT_CE = 0 plain FMNMX pairs, otherwise kSelectMix

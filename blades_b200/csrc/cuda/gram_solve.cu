@@ -7,6 +7,9 @@
 // graphs).  Here each solver is one small fp64 kernel that turns G into the weight vector w (fp32, device memory) that
 // row_combine reads directly: the aggregation path Gram -> (in-switch reduce) -> solve -> combine has no host sync.
 //
+// The Min-Max / Min-Sum scale search (attackers/_agr.py::gram_scale is its host twin) runs here as well: it leaves the
+// scale and the parameter of the malicious virtual row in device memory, where the select and attack-row kernels read it.
+//
 // The arithmetic mirrors csrc/host/selectors.cpp statement for statement (same clamps, same stopping rule, stable
 // tie-breaking by index), so both produce the same weights up to fp64 summation order.
 #include "common.cuh"
@@ -38,6 +41,24 @@ __device__ double block_sum(double v, double* red) {
         double t = lane < (int)(blockDim.x >> 5) ? red[lane] : 0.0;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) t += __shfl_down_sync(0xffffffffu, t, o);
+        if (lane == 0) red[0] = t;
+    }
+    __syncthreads();
+    return red[0];
+}
+
+// block-wide maximum, result broadcast to every thread
+__device__ double block_max(double v, double* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_down_sync(0xffffffffu, v, o));
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    __syncthreads();
+    if (lane == 0) red[wid] = v;
+    __syncthreads();
+    if (wid == 0) {
+        double t = lane < (int)(blockDim.x >> 5) ? red[lane] : -INFINITY;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) t = fmax(t, __shfl_down_sync(0xffffffffu, t, o));
         if (lane == 0) red[0] = t;
     }
     __syncthreads();
@@ -301,3 +322,80 @@ extern "C" int bl_gram_iter(const IterParams* p, void* stream) {
     return (int)cudaGetLastError();
 }
 extern "C" int bl_sizeof_iter_params() { return (int)sizeof(IterParams); }
+
+// ------------------------------------------------------------------------------------- Min-Max / Min-Sum scale
+// Shejwalkar & Houmansadr (NDSS 2021): the malicious row is m(g) = mu - g * p over the honest rows H, with g the largest
+// scale that passes   minmax: max_i ||m - u_i||^2 <= max_{i,j} ||u_i - u_j||^2
+//                     minsum: sum_i ||m - u_i||^2 <= max_i sum_j ||u_i - u_j||^2.
+// Everything is a function of the Gram matrix of [U; q]:
+//   ||m - u_i||^2 = ||mu - u_i||^2 - 2 g (mu.p - u_i.p) + g^2 ||p||^2,   mu.u_i = mean_j G_ij,  ||mu||^2 = mean_i mu.u_i
+// with p = mu / ||mu|| (unit_vec: no q row, all from G), or p = q (std / sign: q is the extra Gram row).
+// One thread per honest row; the search loop is the authors' bisection, in fp64, capped at 128 iterations.
+struct AgrScaleParams {
+    const float* G; const int* idx; int ld;
+    const int* honest;     // [n_h] logical Gram rows of the honest clients
+    int n_h;
+    int q_row;             // logical Gram row of q (std / sign); -1 for unit_vec
+    int minsum;            // 0 Min-Max, 1 Min-Sum
+    int dev_type;          // 0 unit_vec, 1 std, 2 sign
+    double gamma_init, tol;
+    double* gamma;         // [1] out: the scale
+    float* param;          // [1] out: parameter of the virtual row's kernel form (IPM for unit_vec, ALIE for std, 3 sign)
+};
+
+constexpr int kAgrMaxIter = 128;
+
+__global__ void __launch_bounds__(kSolveThreads)
+gram_agr_scale_kernel(const __grid_constant__ AgrScaleParams p) {
+    __shared__ double red[32];
+    const GramView g{p.G, p.idx, p.ld};
+    const int t = threadIdx.x, nh = p.n_h;
+    const bool live = t < nh;
+    const int i = live ? p.honest[t] : 0;
+    double mui = 0.0, gii = 0.0, rmax = 0.0, rsum = 0.0;
+    if (live) {
+        gii = (double)g.at(i, i);
+        for (int k = 0; k < nh; ++k) {
+            const int j = p.honest[k];
+            const double gij = (double)g.at(i, j);
+            mui += gij;
+            const double d = fmax(gii + (double)g.at(j, j) - 2.0 * gij, 0.0);
+            rmax = fmax(rmax, d);
+            rsum += d;
+        }
+        mui /= nh;
+    }
+    const double mumu = block_sum(live ? mui : 0.0, red) / nh;
+    const double thr = block_max(live ? (p.minsum ? rsum : rmax) : 0.0, red);
+    double up = 0.0, mup = 0.0, pp = 0.0, nrm = 0.0;
+    if (p.dev_type == 0) {
+        nrm = sqrt(fmax(mumu, 0.0));
+        if (nrm > 0.0) { up = mui / nrm; mup = nrm; pp = 1.0; }
+    } else {
+        up = live ? (double)g.at(i, p.q_row) : 0.0;
+        mup = block_sum(up, red) / nh;
+        pp = (double)g.at(p.q_row, p.q_row);
+    }
+    const double d0 = fmax(mumu - 2.0 * mui + gii, 0.0), a = mup - up;
+    double gam = p.gamma_init, step = p.gamma_init, ok = 0.0;
+    for (int it = 0; it < kAgrMaxIter && fabs(ok - gam) > p.tol; ++it) {     // uniform: every value is a broadcast
+        const double di = live ? fmax(d0 - 2.0 * gam * a + gam * gam * pp, 0.0) : 0.0;
+        const double v = p.minsum ? block_sum(di, red) : block_max(di, red);
+        if (v <= thr) { ok = gam; gam += step / 2.0; }
+        else gam -= step / 2.0;
+        step /= 2.0;
+    }
+    if (t == 0) {
+        *p.gamma = ok;
+        *p.param = p.dev_type == 0 ? (nrm > 0.0 ? (float)(ok / nrm - 1.0) : -1.f) : (float)ok;
+    }
+}
+
+extern "C" int bl_gram_agr_scale(const AgrScaleParams* p, void* stream) {
+    if (p->n_h < 1 || p->n_h > kSolveThreads || p->dev_type < 0 || p->dev_type > 2) return -1;
+    if ((p->dev_type != 0) != (p->q_row >= 0)) return -1;
+    if (!(p->gamma_init > 0.0) || !(p->tol > 0.0)) return -1;
+    gram_agr_scale_kernel<<<1, kSolveThreads, 0, (cudaStream_t)stream>>>(*p);
+    return (int)cudaGetLastError();
+}
+extern "C" int bl_sizeof_agr_scale_params() { return (int)sizeof(AgrScaleParams); }

@@ -26,8 +26,12 @@ BL_CORE_FN float bl_sat01(float x) {
 #endif
 }
 
+// sign(x) with sign(0) = 0
+BL_CORE_FN float bl_sign(float x) { return (float)((x > 0.f) - (x < 0.f)); }
+
 // Virtual value from the statistics of the first n_stat values in LOAD order (a[0..H) are rows 0..H-1, b[0..H) rows
-// H..NP-1): kind 1 = ALIE mean - p * std_unbiased, kind 2 = IPM -p * mean (same arithmetic as coord_select_kernel).
+// H..NP-1): kind 1 = ALIE mean - p * std_unbiased, kind 2 = IPM -p * mean, kind 3 = mean - p * sign(mean) (Min-Max /
+// Min-Sum with the sign deviation; same arithmetic as coord_select_kernel).
 template <int NP>
 BL_CORE_FN float bl_virtual_value(const float (&a)[NP / 2], const float (&b)[NP / 2], int n_stat, int kind, float param) {
     constexpr int H = NP / 2;
@@ -38,6 +42,7 @@ BL_CORE_FN float bl_virtual_value(const float (&a)[NP / 2], const float (&b)[NP 
 #pragma unroll
     for (int i = 0; i < H; ++i) s = fmaf(b[i], bl_sat01(fstat - (float)(H + i)), s);
     const float mu = s / fstat;
+    if (kind == 3) return mu - param * bl_sign(mu);
     if (kind != 1) return -param * mu;
     float q = 0.f;
 #pragma unroll
@@ -64,6 +69,7 @@ template <int NP>
 BL_CORE_FN float bl_virtual_value_all(const float (&a)[NP / 2], const float (&b)[NP / 2], float total, int kind, float param) {
     constexpr int H = NP / 2;
     const float mu = total / (float)NP;
+    if (kind == 3) return mu - param * bl_sign(mu);
     if (kind != 1) return -param * mu;
     float q0 = 0.f, q1 = 0.f;
 #pragma unroll

@@ -175,7 +175,9 @@ def _default_ce(fn) -> bool:
 def _fusable_classes():
     from ..attackers.alieclient import AlieClient
     from ..attackers.ipmclient import IpmClient
-    return (AlieClient, IpmClient)
+    from ..attackers.minmaxclient import MinmaxClient
+    from ..attackers.minsumclient import MinsumClient
+    return (AlieClient, IpmClient, MinmaxClient, MinsumClient)
 
 
 class RoundEngine:
@@ -555,7 +557,8 @@ class RoundEngine:
 
     def _stock_types(self, rows: List[int]) -> bool:
         from .. import attackers as A
-        stock = (BladesClient, A.NoiseClient, A.LabelflippingClient, A.SignflippingClient, A.AlieClient, A.IpmClient)
+        stock = (BladesClient, A.NoiseClient, A.LabelflippingClient, A.SignflippingClient, A.AlieClient, A.IpmClient,
+                 A.MinmaxClient, A.MinsumClient)
         return all(type(self.clients[self.local_idx[r]]) in stock for r in rows)
 
     def _train_batched(self, rows: List[int], lr: float) -> None:
@@ -1007,7 +1010,7 @@ class RoundEngine:
 
     # ------------------------------------------------------------------ attack phase
     def fusable_attack(self, callbacks: Sequence[Callable]) -> Optional[VirtualRows]:
-        """If every registered omniscient callback belongs to a stock ALIE/IPM client with
+        """If every registered omniscient callback belongs to a stock ALIE / IPM / Min-Max / Min-Sum client with
         identical parameters, describe the attack as virtual rows."""
         if not callbacks:
             return None
@@ -1022,7 +1025,8 @@ class RoundEngine:
             if spec is None or not stock:
                 return None
             owners.append((owner, spec))
-        kinds = {(s["kind"], round(s["param"], 12)) for _, s in owners}
+        kinds = {(s["kind"], round(s["param"], 12), s.get("dev_type"), s.get("gamma_init"), s.get("tol"))
+                 for _, s in owners}
         if len(kinds) != 1:
             return None
         idx_of = {id(c): i for i, c in enumerate(self.clients)}
@@ -1030,8 +1034,16 @@ class RoundEngine:
         if len(replaced) != len(owners):
             return None
         byz = [i for i, c in enumerate(self.clients) if c.is_byzantine()]
-        kind, param = owners[0][1]["kind"], owners[0][1]["param"]
-        return VirtualRows(kind, param, replaced, byz)
+        spec = owners[0][1]
+        if spec["kind"] in ("minmax", "minsum"):
+            clients = [o for o, _ in owners]
+
+            def report(gamma):              # every attacker's ``gamma`` property reads the last scale
+                for o in clients:
+                    o._set_gamma(gamma)
+            return VirtualRows(spec["kind"], spec["param"], replaced, byz, dev_type=spec["dev_type"],
+                               gamma_init=spec["gamma_init"], tol=spec["tol"], report=report)
+        return VirtualRows(spec["kind"], spec["param"], replaced, byz)
 
     # ------------------------------------------------------------------ aggregation
     def make_matrix(self, virtual: Optional[VirtualRows] = None) -> UpdateMatrix:

@@ -13,7 +13,7 @@ import torch
 from . import _loader
 
 __all__ = ["DeviceGram", "enabled", "krum_weights", "weiszfeld_weights", "centered_clip_coeffs", "fltrust_weights",
-           "autogm_weights"]
+           "autogm_weights", "agr_scale"]
 
 
 def enabled() -> bool:
@@ -47,6 +47,12 @@ class IterParams(C.Structure):
                 ("tau", C.c_double), ("alphas", C.c_void_p), ("gs", C.c_void_p), ("use_smem", C.c_int),
                 ("w", C.c_void_p), ("iters", C.c_void_p), ("lamb", C.c_double), ("sort_by_index", C.c_int),
                 ("pad_", C.c_int)]
+
+
+class AgrScaleParams(C.Structure):
+    _fields_ = [("G", C.c_void_p), ("idx", C.c_void_p), ("ld", C.c_int), ("honest", C.c_void_p), ("n_h", C.c_int),
+                ("q_row", C.c_int), ("minsum", C.c_int), ("dev_type", C.c_int), ("gamma_init", C.c_double),
+                ("tol", C.c_double), ("gamma", C.c_void_p), ("param", C.c_void_p)]
 
 
 class TrustParams(C.Structure):
@@ -161,3 +167,25 @@ def fltrust_weights(dg: DeviceGram, trusted: int, eps: float = 1e-6) -> torch.Te
     _loader.check(lib.bl_gram_fltrust(C.byref(p), _loader.stream_ptr(dev)), "gram_fltrust")
     _loader.count_launch()
     return w
+
+
+def agr_scale(dg: DeviceGram, honest: torch.Tensor, q_row: int, minsum: bool, dev_type: str, gamma_init: float,
+              tol: float) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Min-Max / Min-Sum scale search on the Gram matrix of ``[U; q]`` (``honest``: int32 device tensor of the honest
+    logical rows; ``q_row``: logical row of q, -1 for ``unit_vec``).  Returns ``(gamma, param)``: a float64 and a
+    float32 one-element device tensor, ``param`` being the parameter of the virtual row's kernel form."""
+    from .attack import DEV_TYPE
+    lib = _lib()
+    assert lib.bl_sizeof_agr_scale_params() == C.sizeof(AgrScaleParams)
+    dev = dg.G.device
+    gamma = torch.empty(1, dtype=torch.float64, device=dev)
+    param = torch.empty(1, dtype=torch.float32, device=dev)
+    p = AgrScaleParams()
+    p.G, p.idx, p.ld = dg.G.data_ptr(), dg.idx.data_ptr(), dg.G.stride(0)
+    p.honest, p.n_h, p.q_row = honest.data_ptr(), honest.numel(), int(q_row)
+    p.minsum, p.dev_type = int(bool(minsum)), DEV_TYPE[dev_type]
+    p.gamma_init, p.tol = float(gamma_init), float(tol)
+    p.gamma, p.param = gamma.data_ptr(), param.data_ptr()
+    _loader.check(lib.bl_gram_agr_scale(C.byref(p), _loader.stream_ptr(dev)), "gram_agr_scale")
+    _loader.count_launch()
+    return gamma, param

@@ -1,5 +1,5 @@
 """Launchers for the coordinate-select kernels (csrc/cuda/coord_select.cu):
-trimmed mean / median over client rows with optional fused ALIE/IPM virtual rows and the
+trimmed mean / median over client rows with optional fused ALIE/IPM/sign virtual rows and the
 replicated-store + server-step epilogue.  Rows are given as raw device pointers so the same
 launcher serves one dense matrix and NVLink peer shards."""
 from __future__ import annotations
@@ -13,7 +13,7 @@ from . import _loader, _structs
 
 __all__ = ["trimmed_mean", "median", "launch_select", "row_pointers", "make_epilogue"]
 
-_KIND = {None: 0, "alie": 1, "ipm": 2}
+_KIND = {None: 0, "alie": 1, "ipm": 2, "sign": 3}
 
 
 def row_pointers(data: torch.Tensor, rows: Optional[Sequence[int]] = None) -> List[int]:
@@ -44,10 +44,12 @@ def make_epilogue(outs: Sequence[int], thetas: Sequence[int] = (), theta_src: in
 
 def launch_select(stat_rows: Sequence[int], other_rows: Sequence[int], n_virtual: int, kind: Optional[str],
                   param: float, mode: int, trim_b: int, c0: int, c1: int, ep: _structs.Epilogue,
-                  device=None) -> None:
-    """``stat_rows`` (pointers) enter the attack statistics; ``other_rows`` are real rows that do not."""
+                  device=None, param_ptr: int = 0) -> None:
+    """``stat_rows`` (pointers) enter the attack statistics; ``other_rows`` are real rows that do not.
+    ``param_ptr``: address of a device float32 the kernel reads instead of ``param`` (the scale solver's output)."""
     lib = _loader.cuda_lib()
     p, fn = _select_params(lib, stat_rows, other_rows, n_virtual, kind, param, mode, trim_b, c0, c1, ep)
+    p.virt_param_ptr = (param_ptr or None) if n_virtual else None
     _loader.check(fn(C.byref(p), _loader.stream_ptr(device)), "coord_select")
     _loader.count_launch()
 
@@ -95,7 +97,7 @@ def _dense(data: torch.Tensor, mode: int, b: int, virtual) -> torch.Tensor:
         stat = row_pointers(data, [i for i in range(n) if i not in byz])
         other = row_pointers(data, [i for i in range(n) if i in byz and i not in rep])
         launch_select(stat, other, virtual.count, virtual.kind, virtual.param, mode, b, 0, d,
-                      make_epilogue([out.data_ptr()]), data.device)
+                      make_epilogue([out.data_ptr()]), data.device, param_ptr=virtual.param_ptr())
     else:
         launch_select(row_pointers(data), [], 0, None, 0.0, mode, b, 0, d,
                       make_epilogue([out.data_ptr()]), data.device)

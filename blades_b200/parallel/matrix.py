@@ -23,25 +23,34 @@ Primitives (everything the 11 reference aggregators need, SURVEY 2.7 K2-K6):
 
 *Virtual rows* (SURVEY 7.2.3): a ``VirtualRows`` spec replaces the first ``f``
 rows by a coordinate-wise closed form of the honest rows (ALIE / IPM), so the
-fused kernels never store f identical malicious rows.
+fused kernels never store f identical malicious rows.  Min-Max / Min-Sum rows are
+such a closed form with a scale found by a search over pairwise distances; the
+search runs on the Gram matrix of ``[U; q]`` before the first primitive
+(``resolve_scaled_rows``).
 """
 from __future__ import annotations
 
 from dataclasses import dataclass, field
-from typing import Optional, Sequence
+from typing import Callable, Optional, Sequence
 
 import numpy as np
 import torch
 
-__all__ = ["VirtualRows", "UpdateMatrix", "LocalMatrix", "as_matrix"]
+__all__ = ["VirtualRows", "UpdateMatrix", "LocalMatrix", "as_matrix", "resolve_scaled_rows", "SCALED_KINDS"]
+
+#: virtual-row kinds whose value needs a scale search over the whole vector (attackers/_agr.py)
+SCALED_KINDS = ("minmax", "minsum")
 
 
 @dataclass
 class VirtualRows:
     """``count`` identical rows ``value(honest rows)`` replacing rows ``replaced``.
 
-    kind='alie': value = mean - z * std_unbiased   (reference alieclient.py:32-36)
-    kind='ipm' : value = -eps * mean               (reference ipmclient.py:16)
+    kind='alie'  : value = mean - z * std_unbiased   (reference alieclient.py:32-36)
+    kind='ipm'   : value = -eps * mean               (reference ipmclient.py:16)
+    kind='sign'  : value = mean - param * sign(mean)
+    kind='minmax' / 'minsum': value = mean - gamma * p, ``p`` given by ``dev_type`` and ``gamma`` found by the
+                   Min-Max / Min-Sum search (attackers/_agr.py; ``param`` is unused)
     Honest rows = all rows whose index is not in ``byzantine`` (all Byzantine rows,
     not only the replaced ones, are excluded from the statistics).
     """
@@ -49,10 +58,20 @@ class VirtualRows:
     param: float
     replaced: Sequence[int]
     byzantine: Sequence[int] = field(default_factory=list)
+    dev_type: str = "unit_vec"
+    gamma_init: float = 10.0
+    tol: float = 1e-5
+    #: float32 one-element device tensor the kernels read instead of ``param`` (left there by the scale solver)
+    param_dev: Optional[torch.Tensor] = field(default=None, repr=False)
+    #: minmax / minsum: called with the scale of every evaluation (a float, or a float64 one-element device tensor)
+    report: Optional[Callable] = field(default=None, repr=False, compare=False)
 
     def __post_init__(self):
-        if self.kind not in ("alie", "ipm"):
+        if self.kind not in ("alie", "ipm", "sign") + SCALED_KINDS:
             raise ValueError(self.kind)
+        if self.kind in SCALED_KINDS:
+            from ..attackers import _agr
+            _agr.check_args(self.kind, self.dev_type, self.gamma_init, self.tol)
         if not self.byzantine:
             self.byzantine = list(self.replaced)
 
@@ -60,11 +79,67 @@ class VirtualRows:
     def count(self) -> int:
         return len(self.replaced)
 
+    def param_ptr(self) -> int:
+        return self.param_dev.data_ptr() if self.param_dev is not None else 0
+
     def value(self, honest: torch.Tensor) -> torch.Tensor:
+        if self.kind in SCALED_KINDS:
+            from ..attackers import _agr
+            gamma, m = _agr.direct_scale(honest, self.kind, self.dev_type, self.gamma_init, self.tol)
+            if self.report is not None:
+                self.report(gamma)
+            return m.to(honest.dtype)
+        param = self.param if self.param_dev is None else float(self.param_dev)
         mu = honest.mean(dim=0)
         if self.kind == "alie":
-            return mu - self.param * honest.std(dim=0, unbiased=True)
-        return -self.param * mu
+            return mu - param * honest.std(dim=0, unbiased=True)
+        if self.kind == "sign":
+            return mu - param * torch.sign(mu)
+        return -param * mu
+
+
+def resolve_scaled_rows(matrix: "UpdateMatrix") -> None:
+    """Min-Max / Min-Sum virtual rows -> the closed form the kernels evaluate, before the first primitive reads them.
+
+    The scale depends on every coordinate, so it is found once for the whole vector: the deviation pass writes
+    ``q`` (std or sign(mean) of the honest rows; ``unit_vec`` needs no pass, ``mean . u_i`` is a row mean of the
+    Gram), one Gram pass covers ``[U; q]`` and the scale solver turns it into the parameter of an ALIE (std), IPM
+    (unit_vec) or sign form (``attackers._agr.KERNEL_FORM``), left in device memory.  When the Gram cannot stay on
+    the device (CPU, fp32 Gram precision, solvers disabled) the same search runs on the host on ``gram()``.
+    ``matrix.virtual`` is replaced by the resolved form; other kinds are left alone."""
+    v = matrix.virtual
+    if v is None or not v.count or v.kind not in SCALED_KINDS:
+        return
+    from ..attackers import _agr
+    if matrix.window is not None:
+        raise ValueError(f"{v.kind} virtual rows depend on every coordinate and cannot be aggregated window by window")
+    n = matrix.n_rows
+    byz = set(v.byzantine)
+    honest = [i for i in range(n) if i not in byz]
+    _agr.check_honest(len(honest), v.dev_type)
+    use_q = v.dev_type != "unit_vec"
+    blocks = matrix.gram_block_rows() + ([1] if use_q else [])
+    padded = sum((r + 7) // 8 * 8 for r in blocks)
+    if padded > 512 or len(blocks) > 9:
+        raise ValueError(f"{v.kind} with dev_type={v.dev_type!r} needs one Gram pass over the {n} client rows"
+                         f"{' plus the deviation row' if use_q else ''}: {padded} padded rows in {len(blocks)} blocks, "
+                         f"but the Gram pass takes at most 512 padded rows in 9 blocks")
+    matrix.virtual = None                    # the Gram below is of the clients' own rows
+    q = matrix.deviation_row(honest, v.dev_type) if use_q else None
+    q_row = n if use_q else -1
+    dg = matrix.gram_device(extra=q)
+    form = _agr.KERNEL_FORM[v.dev_type]
+    if dg is not None:
+        from ..ops import gram_solve
+        gamma, param = gram_solve.agr_scale(dg, gram_solve.index_tensor(honest, matrix.device), q_row,
+                                            v.kind == "minsum", v.dev_type, v.gamma_init, v.tol)
+        resolved = VirtualRows(form, 0.0, v.replaced, v.byzantine, param_dev=param)
+    else:
+        gamma, param = _agr.gram_scale(matrix.gram(extra=q), honest, q_row, v.kind, v.dev_type, v.gamma_init, v.tol)
+        resolved = VirtualRows(form, param, v.replaced, v.byzantine)
+    if v.report is not None:
+        v.report(gamma)
+    matrix.virtual = resolved
 
 
 class UpdateMatrix:
@@ -105,6 +180,15 @@ class UpdateMatrix:
         """The Gram matrix left ON THE DEVICE (``ops.gram_solve.DeviceGram``) for the on-device solvers, or ``None``
         when this matrix has no kernel path (CPU oracle): callers then fall back to ``gram()`` + the host solvers."""
         return None
+
+    def gram_block_rows(self) -> list:
+        """Row count of every block the Gram pass reads (each is padded to 8 rows)."""
+        from ..ops._gram_impl import split_blocks
+        return [b[2] for b in split_blocks(0, 0, self.n_rows)]
+
+    def deviation_row(self, honest: Sequence[int], dev_type: str) -> torch.Tensor:
+        """The Min-Max / Min-Sum deviation vector q over the rows ``honest`` (``[n_cols]`` float32)."""
+        raise NotImplementedError
     # escape hatch ----------------------------------------------------------------
     def rows(self) -> torch.Tensor: raise NotImplementedError
 
@@ -142,17 +226,28 @@ class LocalMatrix(UpdateMatrix):
         keep = [i for i in range(self.n_rows) if i not in set(v.byzantine)]
         return self.data[keep]
 
+    def deviation_row(self, honest: Sequence[int], dev_type: str) -> torch.Tensor:
+        if not self.use_kernels:
+            from ..attackers import _agr
+            return _agr.deviation(torch.nan_to_num(self.data[list(honest)]), dev_type).to(torch.float32)
+        from ..ops import attack as _a, select as _s
+        q = torch.empty(self.n_cols, device=self.device, dtype=torch.float32)
+        _a.deviation(_s.row_pointers(self.data, honest), dev_type, 0, self.n_cols, q, self.device)
+        return q
+
     def materialize_virtual(self) -> torch.Tensor:
         """Write the virtual rows into ``data`` (what the reference's callbacks do)."""
         v = self.virtual
         if v is not None and v.count:
             if self.use_kernels:
                 from ..ops import attack as _a, select as _s
+                resolve_scaled_rows(self)
+                v = self.virtual
                 byz = set(v.byzantine)
                 honest = [i for i in range(self.n_rows) if i not in byz]
                 c0, c1 = self._cols()
                 _a.attack_rows(_s.row_pointers(self.data, honest), _s.row_pointers(self.data, list(v.replaced)),
-                               v.kind, v.param, c0, c1, self.data.device)
+                               v.kind, v.param, c0, c1, self.data.device, param_ptr=v.param_ptr())
             else:
                 val = v.value(self._honest())
                 self.data[list(v.replaced)] = val
@@ -239,6 +334,7 @@ class LocalMatrix(UpdateMatrix):
 
     def _select_kernel(self, mode: int, b: int) -> torch.Tensor:
         from ..ops import select as _s
+        resolve_scaled_rows(self)
         data, v, n = self.data, self.virtual, self.n_rows
         out = self._out(data.device)
         c0, c1 = self._cols()
@@ -247,7 +343,7 @@ class LocalMatrix(UpdateMatrix):
             stat = _s.row_pointers(data, [i for i in range(n) if i not in byz])
             other = _s.row_pointers(data, [i for i in range(n) if i in byz and i not in rep])
             _s.launch_select(stat, other, v.count, v.kind, v.param, mode, b, c0, c1,
-                             self._epilogue(out), data.device)
+                             self._epilogue(out), data.device, param_ptr=v.param_ptr())
         else:
             _s.launch_select(_s.row_pointers(data), [], 0, None, 0.0, mode, b, c0, c1,
                              self._epilogue(out), data.device)

@@ -27,7 +27,7 @@ import torch.distributed as dist
 from ..ops import attack as k_attack
 from ..ops import combine as k_combine
 from ..ops import select as k_select
-from .matrix import UpdateMatrix, VirtualRows
+from .matrix import UpdateMatrix, VirtualRows, resolve_scaled_rows
 
 __all__ = ["ShardedMatrix"]
 
@@ -171,21 +171,38 @@ class ShardedMatrix(UpdateMatrix):
             self.symm.barrier()          # every shard of agg/theta has landed everywhere
         return self.symm.agg
 
+    def gram_block_rows(self) -> list:
+        from ..ops import _gram_impl
+        return [b[2] for (ptr, ld, rows) in self.symm.block_descs() for b in _gram_impl.split_blocks(ptr, ld, rows)]
+
+    def deviation_row(self, honest, dev_type: str) -> torch.Tensor:
+        """q over this rank's coordinates only (the Gram pass of this rank reads no others); the rows are pulled from
+        their owners, as the select kernels do."""
+        self.push = False                # the Gram pass that follows pulls the rows of U itself
+        self._pre()
+        q = torch.zeros(self.n_cols, device=self.device, dtype=torch.float32)
+        c0, c1 = self._cols()
+        k_attack.deviation(self._ptrs(honest), dev_type, c0, c1, q, self.device)
+        return q
+
     def materialize_virtual(self):
         v = self.virtual
         if v is not None and v.count:
+            resolve_scaled_rows(self)
+            v = self.virtual
             self._pre()
             s = self.symm
             byz = set(v.byzantine)
             honest = [i for i in range(self.n_rows) if i not in byz]
             c0, c1 = self._cols()
             k_attack.attack_rows(self._ptrs(honest), self._ptrs(list(v.replaced)), v.kind, v.param, c0, c1,
-                                 self.device)
+                                 self.device, param_ptr=v.param_ptr())
             self.virtual = None
             self._barrier()
 
     # ------------------------------------------------------------------ primitives
     def _select(self, mode: int, b: int) -> torch.Tensor:
+        resolve_scaled_rows(self)
         self._pre()
         s = self.symm
         c0, c1 = self._cols()
@@ -195,7 +212,7 @@ class ShardedMatrix(UpdateMatrix):
             stat = self._ptrs([i for i in range(self.n_rows) if i not in byz])
             other = self._ptrs([i for i in range(self.n_rows) if i in byz and i not in rep])
             k_select.launch_select(stat, other, v.count, v.kind, v.param, mode, b, c0, c1,
-                                   self._epilogue(True), self.device)
+                                   self._epilogue(True), self.device, param_ptr=v.param_ptr())
         else:
             k_select.launch_select(self._ptrs(range(self.n_rows)), [], 0, None, 0.0, mode, b, c0, c1,
                                    self._epilogue(True), self.device)

@@ -32,13 +32,13 @@ from .client import BladesClient, ByzantineClient
 from .comm.group import World, get_world
 from .datasets.dataset import FLDataset
 from .engine.round import RoundEngine
-from .parallel.matrix import VirtualRows
+from .parallel.matrix import SCALED_KINDS, VirtualRows
 from .server import BladesServer
 from .utils import initialize_logger, reset_model_weights, set_random_seed, top1_accuracy
 
 __all__ = ["Simulator"]
 
-BUILTIN_ATTACKS = ("noise", "labelflipping", "signflipping", "alie", "ipm")
+BUILTIN_ATTACKS = ("noise", "labelflipping", "signflipping", "alie", "ipm", "minmax", "minsum")
 
 
 class _NullBar:
@@ -366,11 +366,20 @@ class Simulator(object):
         from .ops import gram_solve
         devsolve = type(self.aggregator) in (Krum, Multikrum, Geomed, Autogm, Centeredclipping, Fltrust) and gram_solve.enabled() \
             and eng.use_kernels
-        eng.agg_windows_ok = coordwise          # only coordinate-wise aggregators can be pipelined window by window
+        virtual = self._cached_virtual() if self._active_callbacks() else None
+        # only coordinate-wise aggregators can be pipelined window by window, and only when the attack is
+        # coordinate-wise as well: the Min-Max / Min-Sum scale depends on every coordinate
+        scaled = virtual is not None and virtual.kind in SCALED_KINDS
+        eng.agg_windows_ok = coordwise and not scaled
         if not (coordwise or devsolve) or not self.server._flat_fast_path_ok():
             return False
-        if self._active_callbacks() and self._cached_virtual() is None:
+        if self._active_callbacks() and virtual is None:
             return False
+        if scaled:
+            # the scale search must stay on the device (a host solve syncs, and a capture fails on a sync)
+            from .ops import gram as _gram
+            if not (gram_solve.enabled() and eng.use_kernels and _gram.PRECISION != "fp32"):
+                return False
         return eng.all_rows_static()
 
     def train_trainer(self, epoch, num_rounds, clients):
