@@ -1046,17 +1046,17 @@ class RoundEngine:
         return VirtualRows(spec["kind"], spec["param"], replaced, byz)
 
     # ------------------------------------------------------------------ aggregation
-    def make_matrix(self, virtual: Optional[VirtualRows] = None) -> UpdateMatrix:
+    def make_matrix(self, virtual: Optional[VirtualRows] = None, window=None, chunk: int = 0, last: bool = True,
+                    out: Optional[torch.Tensor] = None, recv_col: int = 0) -> UpdateMatrix:
+        """``window`` / ``chunk`` / ``last`` / ``out`` / ``recv_col``: pipelined aggregation (``_AggPipeline``) -- the
+        matrix covers coordinates ``[window[0], window[1])`` only; see ``UpdateMatrix.window``."""
         if self.symm is not None:
             from ..parallel.sharded import ShardedMatrix
-            return ShardedMatrix(self.symm, virtual=virtual)
-        if self.world.distributed:
-            # no symmetric memory (CPU / gloo): gather the rows; every rank aggregates identically
-            dense = self.gather_dense()
-            return LocalMatrix(dense, virtual=virtual, use_kernels=self.use_kernels and dense.is_cuda,
-                               theta=self.gflat.theta)
-        return LocalMatrix(self.U, virtual=virtual, use_kernels=self.use_kernels and self.U.is_cuda,
-                           theta=self.gflat.theta)
+            return ShardedMatrix(self.symm, virtual, window=window, chunk=chunk, last_chunk=last, recv_col=recv_col)
+        # no symmetric memory (CPU / gloo): gather the rows; every rank aggregates identically
+        U = self.gather_dense()
+        return LocalMatrix(U, virtual, use_kernels=self.use_kernels and U.is_cuda, theta=self.gflat.theta,
+                           window=window, chunk=chunk, last_chunk=last, out_buffer=out)
 
     def gather_dense(self) -> torch.Tensor:
         """Dense [N, d] on every rank (escape hatch for custom callbacks/aggregators)."""

@@ -52,42 +52,56 @@ def split_blocks(ptr: int, ld: int, rows: int, max_rows: int = 256) -> List[Tupl
     return out
 
 
-def gram_tcgen05(lib, data: torch.Tensor, extra: Optional[torch.Tensor], precision: str) -> Optional[torch.Tensor]:
-    r = gram_padded(lib, data, extra, precision)
-    if r is None:
-        return None
-    out, idx = r
-    idx_t = torch.tensor(idx, device=data.device)
-    G = out[idx_t][:, idx_t]
-    return 0.5 * (G + G.T)
+#: one Gram pass reads at most this many rows (each block padded to 8) in at most this many blocks
+MAX_PADDED_ROWS = 512
+MAX_BLOCKS = 9
 
 
-def gram_padded(lib, data: torch.Tensor, extra: Optional[torch.Tensor], precision: str):
-    """(padded accumulators ``[tile_rows, ld]``, logical -> padded row list) or None when the kernel does not apply."""
-    n, d = data.shape
-    if data.stride(1) != 1 or data.stride(0) % 4 != 0 or data.data_ptr() % 16 != 0:
+def padded_rows(row_counts: Sequence[int]) -> int:
+    return sum(_pad8(r) for r in row_counts)
+
+
+def gram_pass(blocks: Sequence[Tuple[int, int, int]], d: int, col0: int, col1: int, device,
+              extra: Optional[torch.Tensor] = None, split3: bool = True, tf32_fallback: bool = False,
+              scratch: Optional[torch.Tensor] = None):
+    """One Gram pass over the row blocks ``(base_ptr, ld_floats, rows)`` (+ the rows of ``extra``, ``[e, d]``) and
+    coordinates ``[col0, col1)``.  Returns (padded accumulators ``[tile_rows, ld]``, logical -> padded row list), or
+    None when the kernel does not apply: unaligned blocks, more rows or blocks than one pass takes, or -- unless
+    ``tf32_fallback``, which relaunches in plain tf32 -- 3xTF32 staging that does not fit.  The accumulators are a
+    zeroed view of ``scratch`` when given, a new zeroed tensor otherwise."""
+    if any(ptr % 16 or ld % 4 for ptr, ld, _ in blocks):
         return None
-    blocks = split_blocks(data.data_ptr(), data.stride(0), n)
-    e = 0
-    keep = [data]
+    blocks = [b for blk in blocks for b in split_blocks(*blk)]
+    buf = None
     if extra is not None:
         extra = extra.reshape(-1, d)
-        e = extra.shape[0]
-        ld = (d + 3) // 4 * 4
-        buf = torch.zeros(e, ld, device=data.device, dtype=torch.float32)
+        ld = blocks[0][1]
+        buf = torch.zeros(extra.shape[0], ld, device=device, dtype=torch.float32)
         buf[:, :d] = extra
-        keep.append(buf)
-        blocks += split_blocks(buf.data_ptr(), ld, e)
-    total_pad = sum(_pad8(b[2]) for b in blocks)
-    if total_pad > 512 or len(blocks) > 9:
+        blocks += split_blocks(buf.data_ptr(), ld, extra.shape[0])
+    total_pad = padded_rows([b[2] for b in blocks])
+    if total_pad > MAX_PADDED_ROWS or len(blocks) > MAX_BLOCKS:
         return None
     tile_rows = (total_pad + 127) // 128 * 128
     ldg = (total_pad + 31) // 32 * 32
-    out = torch.zeros(tile_rows, ldg, device=data.device, dtype=torch.float32)
-    starts = launch_gram(blocks, d, 0, d, out, precision == "tf32x3", data.device)
+    if scratch is None:
+        out = torch.zeros(tile_rows, ldg, device=device, dtype=torch.float32)
+    else:
+        out = scratch[: tile_rows * ldg].view(tile_rows, ldg)
+        out.zero_()
+    starts = launch_gram(blocks, d, col0, col1, out, split3, device)
+    if starts is None and tf32_fallback:
+        starts = launch_gram(blocks, d, col0, col1, out, False, device)
     if starts is None:
         return None
     idx = []
-    for (ptr, ld, rows), s in zip(blocks, starts):
+    for (_, _, rows), s in zip(blocks, starts):
         idx += list(range(s, s + rows))
     return out, idx
+
+
+def symmetrised(out: torch.Tensor, idx: Sequence[int]) -> torch.Tensor:
+    """The logical ``[n, n]`` Gram ``out[idx][:, idx]`` of a pass's padded accumulators, symmetrised."""
+    idx_t = torch.tensor(idx, device=out.device)
+    G = out[idx_t][:, idx_t]
+    return 0.5 * (G + G.T)

@@ -20,11 +20,13 @@ def gram(data: torch.Tensor, extra: Optional[torch.Tensor] = None, precision: Op
     precision = precision or PRECISION
     from . import _loader
     lib = _loader.cuda_lib()
-    if precision != "fp32" and hasattr(lib, "bl_gram_tcgen05") and data.dtype == torch.float32:
-        from ._gram_impl import gram_tcgen05
-        G = gram_tcgen05(lib, data, extra, precision)
-        if G is not None:
-            return G.double().cpu().numpy()
+    if precision != "fp32" and hasattr(lib, "bl_gram_tcgen05") and data.dtype == torch.float32 \
+            and data.stride(1) == 1:
+        from ._gram_impl import gram_pass, symmetrised
+        n, d = data.shape
+        r = gram_pass([(data.data_ptr(), data.stride(0), n)], d, 0, d, data.device, extra, precision == "tf32x3")
+        if r is not None:
+            return symmetrised(*r).double().cpu().numpy()
     full = data if extra is None else torch.cat([data, extra.reshape(-1, data.shape[1])], 0)
     full = torch.nan_to_num(full)
     prev = torch.backends.cuda.matmul.allow_tf32

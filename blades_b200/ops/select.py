@@ -92,12 +92,10 @@ def _dense(data: torch.Tensor, mode: int, b: int, virtual) -> torch.Tensor:
     n, d = data.shape
     out = torch.empty(d, device=data.device, dtype=torch.float32)
     if virtual is not None and virtual.count:
-        byz = set(virtual.byzantine)
-        rep = set(virtual.replaced)
-        stat = row_pointers(data, [i for i in range(n) if i not in byz])
-        other = row_pointers(data, [i for i in range(n) if i in byz and i not in rep])
-        launch_select(stat, other, virtual.count, virtual.kind, virtual.param, mode, b, 0, d,
-                      make_epilogue([out.data_ptr()]), data.device, param_ptr=virtual.param_ptr())
+        honest, other = virtual.partition(n)
+        launch_select(row_pointers(data, honest), row_pointers(data, other), virtual.count, virtual.kind,
+                      virtual.param, mode, b, 0, d, make_epilogue([out.data_ptr()]), data.device,
+                      param_ptr=virtual.param_ptr())
     else:
         launch_select(row_pointers(data), [], 0, None, 0.0, mode, b, 0, d,
                       make_epilogue([out.data_ptr()]), data.device)

@@ -82,6 +82,12 @@ class VirtualRows:
     def param_ptr(self) -> int:
         return self.param_dev.data_ptr() if self.param_dev is not None else 0
 
+    def partition(self, n: int):
+        """``(honest, other)`` of ``n`` rows: the rows that enter the attack statistics (not Byzantine), and the
+        Byzantine rows that are not replaced (real rows that enter no statistic)."""
+        byz, rep = set(self.byzantine), set(self.replaced)
+        return [i for i in range(n) if i not in byz], [i for i in range(n) if i in byz and i not in rep]
+
     def value(self, honest: torch.Tensor) -> torch.Tensor:
         if self.kind in SCALED_KINDS:
             from ..attackers import _agr
@@ -111,19 +117,20 @@ def resolve_scaled_rows(matrix: "UpdateMatrix") -> None:
     if v is None or not v.count or v.kind not in SCALED_KINDS:
         return
     from ..attackers import _agr
+    from ..ops import _gram_impl
     if matrix.window is not None:
         raise ValueError(f"{v.kind} virtual rows depend on every coordinate and cannot be aggregated window by window")
     n = matrix.n_rows
-    byz = set(v.byzantine)
-    honest = [i for i in range(n) if i not in byz]
+    honest, _ = v.partition(n)
     _agr.check_honest(len(honest), v.dev_type)
     use_q = v.dev_type != "unit_vec"
     blocks = matrix.gram_block_rows() + ([1] if use_q else [])
-    padded = sum((r + 7) // 8 * 8 for r in blocks)
-    if padded > 512 or len(blocks) > 9:
+    padded = _gram_impl.padded_rows(blocks)
+    if padded > _gram_impl.MAX_PADDED_ROWS or len(blocks) > _gram_impl.MAX_BLOCKS:
         raise ValueError(f"{v.kind} with dev_type={v.dev_type!r} needs one Gram pass over the {n} client rows"
                          f"{' plus the deviation row' if use_q else ''}: {padded} padded rows in {len(blocks)} blocks, "
-                         f"but the Gram pass takes at most 512 padded rows in 9 blocks")
+                         f"but the Gram pass takes at most {_gram_impl.MAX_PADDED_ROWS} padded rows in "
+                         f"{_gram_impl.MAX_BLOCKS} blocks")
     matrix.virtual = None                    # the Gram below is of the clients' own rows
     q = matrix.deviation_row(honest, v.dev_type) if use_q else None
     q_row = n if use_q else -1
@@ -143,12 +150,19 @@ def resolve_scaled_rows(matrix: "UpdateMatrix") -> None:
 
 
 class UpdateMatrix:
-    """Interface; see module docstring."""
+    """Interface; see module docstring.
+
+    The kernel path of the primitives is written once here, over a few hooks each matrix supplies: ``_ptrs(rows)``
+    (row pointers for a kernel reading coordinates ``_cols()``), ``_pre()`` (before the first launch), ``_epilogue()``
+    (where the result is stored), ``_finish()`` (after the final launch), ``_rows_written()`` (after the virtual rows
+    are written into the rows), ``_gram_blocks()`` and ``_gram_pass(extra)``."""
 
     n_rows: int
     n_cols: int
     device: torch.device
     virtual: Optional[VirtualRows] = None
+    #: False: the primitives are the pure-torch oracle (``LocalMatrix`` only)
+    use_kernels = True
     #: (lr,) -> the final primitive also applies ``theta += lr * agg`` on every replica (K8 fusion)
     server_step = None
     step_applied = False
@@ -163,6 +177,18 @@ class UpdateMatrix:
     def _cols(self):
         return (0, self.n_cols) if self.window is None else (int(self.window[0]), int(self.window[1]))
 
+    # -- hooks ------------------------------------------------------------------
+    def _ptrs(self, rows) -> list: raise NotImplementedError
+    def _pre(self) -> None: pass
+    def _epilogue(self): raise NotImplementedError      # -> (epilogue, result tensor)
+    def _finish(self) -> None: pass
+    def _rows_written(self) -> None: pass
+    def _gram_blocks(self) -> list: raise NotImplementedError  # -> [(base_ptr, ld_floats, rows)] in row order
+
+    def _gram_pass(self, extra: Optional[torch.Tensor]):
+        """``ops._gram_impl.gram_pass`` over ``_gram_blocks()`` (+ ``extra``), or ``None`` without a kernel path."""
+        return None
+
     # coordinate-wise -----------------------------------------------------------
     def mean(self) -> torch.Tensor:
         w = torch.full((self.n_rows,), 1.0 / self.n_rows, dtype=torch.float64)
@@ -170,34 +196,103 @@ class UpdateMatrix:
 
     def combine(self, weights, extra: Optional[torch.Tensor] = None, extra_weight: float = 0.0) -> torch.Tensor:
         """``sum_i w_i U[i] (+ extra_weight * extra)``."""
-        raise NotImplementedError
-    def trimmed_mean(self, b: int) -> torch.Tensor: raise NotImplementedError
-    def median(self) -> torch.Tensor: raise NotImplementedError
+        from ..ops import combine as _k
+        self.materialize_virtual()
+        self._pre()
+        rows = self._ptrs(range(self.n_rows))
+        if torch.is_tensor(weights) and weights.is_cuda:
+            # device-resident weights (on-device Gram solvers): no host copy; with ``extra`` the last weight is its.
+            # ``extra`` is held past the launch: inside a graph capture the replay reads it
+            if extra is not None:
+                self._keep = extra.to(self.device, torch.float32).contiguous()
+                rows = rows + [self._keep.data_ptr()]
+            w = weights.to(torch.float32).contiguous()
+        else:
+            w = [float(x) for x in (weights.tolist() if hasattr(weights, "tolist") else weights)]
+            if extra is not None and extra_weight != 0.0:
+                extra = extra.contiguous()
+                rows, w = rows + [extra.data_ptr()], w + [float(extra_weight)]
+        c0, c1 = self._cols()
+        ep, out = self._epilogue()
+        _k.launch_combine(rows, w, c0, c1, ep, self.device)
+        self._finish()
+        return out
+
+    def trimmed_mean(self, b: int) -> torch.Tensor:
+        if self.n_rows - 2 * b <= 0:
+            raise ValueError(f"trim {b} too large for {self.n_rows} rows")
+        return self._select(0, b)
+
+    def median(self) -> torch.Tensor:
+        return self._select(1, 0)
+
+    def _select(self, mode: int, b: int) -> torch.Tensor:
+        from ..ops import select as _s
+        resolve_scaled_rows(self)
+        self._pre()
+        v = self.virtual
+        if v is not None and v.count:
+            stat, other = v.partition(self.n_rows)
+            count, kind, param, param_ptr = v.count, v.kind, v.param, v.param_ptr()
+        else:
+            stat, other, count, kind, param, param_ptr = range(self.n_rows), [], 0, None, 0.0, 0
+        c0, c1 = self._cols()
+        ep, out = self._epilogue()
+        _s.launch_select(self._ptrs(stat), self._ptrs(other), count, kind, param, mode, b, c0, c1, ep, self.device,
+                         param_ptr=param_ptr)
+        self._finish()
+        return out
+
+    def materialize_virtual(self) -> None:
+        """Write the virtual rows into the rows they replace (what the reference's callbacks do)."""
+        v = self.virtual
+        if v is not None and v.count:
+            from ..ops import attack as _a
+            resolve_scaled_rows(self)
+            v = self.virtual
+            self._pre()
+            honest, _ = v.partition(self.n_rows)
+            c0, c1 = self._cols()
+            _a.attack_rows(self._ptrs(honest), self._ptrs(list(v.replaced)), v.kind, v.param, c0, c1, self.device,
+                           param_ptr=v.param_ptr())
+            self.virtual = None
+            self._rows_written()
+
     # geometry ------------------------------------------------------------------
     def gram(self, extra: Optional[torch.Tensor] = None) -> np.ndarray: raise NotImplementedError
 
     def gram_device(self, extra: Optional[torch.Tensor] = None):
         """The Gram matrix left ON THE DEVICE (``ops.gram_solve.DeviceGram``) for the on-device solvers, or ``None``
         when this matrix has no kernel path (CPU oracle): callers then fall back to ``gram()`` + the host solvers."""
-        return None
+        from ..ops import gram_solve
+        if not gram_solve.enabled():
+            return None
+        r = self._gram_pass(extra)
+        if r is None:
+            return None
+        out, idx = r
+        return gram_solve.DeviceGram(out, gram_solve.index_tensor(idx, self.device), len(idx))
 
     def gram_block_rows(self) -> list:
         """Row count of every block the Gram pass reads (each is padded to 8 rows)."""
         from ..ops._gram_impl import split_blocks
-        return [b[2] for b in split_blocks(0, 0, self.n_rows)]
+        return [b[2] for blk in self._gram_blocks() for b in split_blocks(*blk)]
 
     def deviation_row(self, honest: Sequence[int], dev_type: str) -> torch.Tensor:
-        """The Min-Max / Min-Sum deviation vector q over the rows ``honest`` (``[n_cols]`` float32)."""
-        raise NotImplementedError
+        """The Min-Max / Min-Sum deviation vector q over the rows ``honest`` (``[n_cols]`` float32), over this
+        matrix's coordinates ``_cols()`` (zero elsewhere)."""
+        from ..ops import attack as _a
+        self._pre()
+        c0, c1 = self._cols()
+        alloc = torch.empty if (c0, c1) == (0, self.n_cols) else torch.zeros
+        q = alloc(self.n_cols, device=self.device, dtype=torch.float32)
+        _a.deviation(self._ptrs(honest), dev_type, c0, c1, q, self.device)
+        return q
     # escape hatch ----------------------------------------------------------------
     def rows(self) -> torch.Tensor: raise NotImplementedError
 
     def __len__(self) -> int:
         return self.n_rows
-
-
-def _sanitize(u: torch.Tensor) -> torch.Tensor:
-    return u
 
 
 class LocalMatrix(UpdateMatrix):
@@ -209,7 +304,8 @@ class LocalMatrix(UpdateMatrix):
     """
 
     def __init__(self, data: torch.Tensor, virtual: Optional[VirtualRows] = None,
-                 use_kernels: Optional[bool] = None, theta: Optional[torch.Tensor] = None):
+                 use_kernels: Optional[bool] = None, theta: Optional[torch.Tensor] = None,
+                 window=None, chunk: int = 0, last_chunk: bool = True, out_buffer: Optional[torch.Tensor] = None):
         assert data.dim() == 2, data.shape
         self.data = data
         self.theta = theta               # flat parameter vector for the fused server step
@@ -219,49 +315,54 @@ class LocalMatrix(UpdateMatrix):
         if use_kernels is None:
             use_kernels = data.is_cuda and data.dtype == torch.float32
         self.use_kernels = use_kernels
+        self.window, self.chunk, self.last_chunk, self.out_buffer = window, chunk, last_chunk, out_buffer
 
-    # -- helpers ------------------------------------------------------------------
-    def _honest(self) -> torch.Tensor:
-        v = self.virtual
-        keep = [i for i in range(self.n_rows) if i not in set(v.byzantine)]
-        return self.data[keep]
+    # -- kernel hooks ---------------------------------------------------------------
+    def _ptrs(self, rows) -> list:
+        from ..ops import select as _s
+        return _s.row_pointers(self.data, rows)
 
+    def _epilogue(self):
+        from ..ops import select as _s
+        out = self.out_buffer
+        if out is None:
+            out = torch.empty(self.n_cols, device=self.device, dtype=torch.float32)
+        if self.server_step is not None and self.theta is not None:
+            self.step_applied = True
+            return _s.make_epilogue([out.data_ptr()], [self.theta.data_ptr()], self.theta.data_ptr(),
+                                    float(self.server_step[0])), out
+        return _s.make_epilogue([out.data_ptr()]), out
+
+    def _gram_blocks(self) -> list:
+        return [(self.data.data_ptr(), self.data.stride(0), self.n_rows)]
+
+    def _gram_pass(self, extra: Optional[torch.Tensor]):
+        from ..ops import _gram_impl, gram as _k
+        if not self.use_kernels or _k.PRECISION == "fp32" or self.rows().stride(1) != 1:
+            return None
+        return _gram_impl.gram_pass(self._gram_blocks(), self.n_cols, 0, self.n_cols, self.device, extra,
+                                    _k.PRECISION == "tf32x3")
+
+    # -- torch oracle (use_kernels=False) ---------------------------------------------
     def deviation_row(self, honest: Sequence[int], dev_type: str) -> torch.Tensor:
-        if not self.use_kernels:
-            from ..attackers import _agr
-            return _agr.deviation(torch.nan_to_num(self.data[list(honest)]), dev_type).to(torch.float32)
-        from ..ops import attack as _a, select as _s
-        q = torch.empty(self.n_cols, device=self.device, dtype=torch.float32)
-        _a.deviation(_s.row_pointers(self.data, honest), dev_type, 0, self.n_cols, q, self.device)
-        return q
+        if self.use_kernels:
+            return super().deviation_row(honest, dev_type)
+        from ..attackers import _agr
+        return _agr.deviation(torch.nan_to_num(self.data[list(honest)]), dev_type).to(torch.float32)
 
     def materialize_virtual(self) -> torch.Tensor:
         """Write the virtual rows into ``data`` (what the reference's callbacks do)."""
         v = self.virtual
-        if v is not None and v.count:
-            if self.use_kernels:
-                from ..ops import attack as _a, select as _s
-                resolve_scaled_rows(self)
-                v = self.virtual
-                byz = set(v.byzantine)
-                honest = [i for i in range(self.n_rows) if i not in byz]
-                c0, c1 = self._cols()
-                _a.attack_rows(_s.row_pointers(self.data, honest), _s.row_pointers(self.data, list(v.replaced)),
-                               v.kind, v.param, c0, c1, self.data.device, param_ptr=v.param_ptr())
-            else:
-                val = v.value(self._honest())
-                self.data[list(v.replaced)] = val
+        if self.use_kernels:
+            super().materialize_virtual()
+        elif v is not None and v.count:
+            val = v.value(self.data[v.partition(self.n_rows)[0]])
+            self.data[list(v.replaced)] = val
             self.virtual = None
         return self.data
 
     def rows(self) -> torch.Tensor:
         return self.materialize_virtual()
-
-    # -- primitives -----------------------------------------------------------------
-    def _out(self, device) -> torch.Tensor:
-        if self.out_buffer is not None:
-            return self.out_buffer
-        return torch.empty(self.n_cols, device=device, dtype=torch.float32)
 
     def _windowed(self, full: torch.Tensor) -> torch.Tensor:
         """CPU oracle of a windowed primitive: the full-width result restricted to this object's window, written into
@@ -274,41 +375,10 @@ class LocalMatrix(UpdateMatrix):
         self.out_buffer[c0:c1] = full[c0:c1]
         return self.out_buffer
 
-    def _epilogue(self, out: torch.Tensor):
-        from ..ops import select as _s
-        if self.server_step is not None and self.theta is not None:
-            self.step_applied = True
-            return _s.make_epilogue([out.data_ptr()], [self.theta.data_ptr()], self.theta.data_ptr(),
-                                    float(self.server_step[0]))
-        return _s.make_epilogue([out.data_ptr()])
-
     def combine(self, weights, extra: Optional[torch.Tensor] = None, extra_weight: float = 0.0) -> torch.Tensor:
-        if self.use_kernels and torch.is_tensor(weights) and weights.is_cuda:
-            # device-resident weights (on-device Gram solvers); with ``extra`` the last weight belongs to it
-            from ..ops import combine as _k, select as _s
-            data = self.rows()
-            rows = _s.row_pointers(data)
-            keep = None
-            if extra is not None:
-                keep = extra.to(data.device, torch.float32).contiguous()
-                rows = rows + [keep.data_ptr()]
-            out = self._out(data.device)
-            c0, c1 = self._cols()
-            _k.launch_combine(rows, weights.to(torch.float32).contiguous(), c0, c1, self._epilogue(out), data.device)
-            return out
-        w = torch.as_tensor(np.asarray(weights, dtype=np.float64) if not torch.is_tensor(weights) else weights)
         if self.use_kernels:
-            from ..ops import combine as _k, select as _s
-            data = self.rows()
-            rows = _s.row_pointers(data)
-            wl = [float(x) for x in w.tolist()]
-            if extra is not None and extra_weight != 0.0:
-                extra = extra.contiguous()
-                rows, wl = rows + [extra.data_ptr()], wl + [float(extra_weight)]
-            out = self._out(data.device)
-            c0, c1 = self._cols()
-            _k.launch_combine(rows, wl, c0, c1, self._epilogue(out), data.device)
-            return out
+            return super().combine(weights, extra, extra_weight)
+        w = torch.as_tensor(np.asarray(weights, dtype=np.float64) if not torch.is_tensor(weights) else weights)
         data = self.rows()
         res = (w.to(data.device, torch.float64)[:, None] * data.double()).sum(0)
         if extra is not None and extra_weight != 0.0:
@@ -320,41 +390,15 @@ class LocalMatrix(UpdateMatrix):
             return super().mean()
         return self._windowed(self.rows().mean(dim=0))
 
-    def trimmed_mean(self, b: int) -> torch.Tensor:
-        n = self.n_rows
-        if n - 2 * b <= 0:
-            raise ValueError(f"trim {b} too large for {n} rows")
+    def _select(self, mode: int, b: int) -> torch.Tensor:
         if self.use_kernels:
-            return self._select_kernel(0, b)
-        data = self.rows()
-        if b == 0:
+            return super()._select(mode, b)
+        data, n = self.rows(), self.n_rows
+        if mode == 0 and b == 0:
             return self._windowed(data.mean(0))
         srt = data.sort(dim=0).values
-        return self._windowed(srt[b: n - b].mean(dim=0))
-
-    def _select_kernel(self, mode: int, b: int) -> torch.Tensor:
-        from ..ops import select as _s
-        resolve_scaled_rows(self)
-        data, v, n = self.data, self.virtual, self.n_rows
-        out = self._out(data.device)
-        c0, c1 = self._cols()
-        if v is not None and v.count:
-            byz, rep = set(v.byzantine), set(v.replaced)
-            stat = _s.row_pointers(data, [i for i in range(n) if i not in byz])
-            other = _s.row_pointers(data, [i for i in range(n) if i in byz and i not in rep])
-            _s.launch_select(stat, other, v.count, v.kind, v.param, mode, b, c0, c1,
-                             self._epilogue(out), data.device, param_ptr=v.param_ptr())
-        else:
-            _s.launch_select(_s.row_pointers(data), [], 0, None, 0.0, mode, b, c0, c1,
-                             self._epilogue(out), data.device)
-        return out
-
-    def median(self) -> torch.Tensor:
-        if self.use_kernels:
-            return self._select_kernel(1, 0)
-        data = self.rows()
-        n = self.n_rows
-        srt = data.sort(dim=0).values
+        if mode == 0:
+            return self._windowed(srt[b: n - b].mean(dim=0))
         return self._windowed((srt[(n - 1) // 2] + srt[n // 2]) * 0.5)
 
     def gram(self, extra: Optional[torch.Tensor] = None) -> np.ndarray:
@@ -367,25 +411,6 @@ class LocalMatrix(UpdateMatrix):
         full = data if extra is None else torch.cat([data, extra], 0)
         full = full.double()
         return (full @ full.T).cpu().numpy()
-
-
-def _local_gram_device(self, extra: Optional[torch.Tensor] = None):
-    if not self.use_kernels:
-        return None
-    from ..ops import _gram_impl, _loader, gram as _k, gram_solve
-    if not gram_solve.enabled() or _k.PRECISION == "fp32":
-        return None
-    data = self.rows()
-    if extra is not None:
-        extra = extra.reshape(-1, self.n_cols).to(data.device, data.dtype)
-    r = _gram_impl.gram_padded(_loader.cuda_lib(), data, extra, _k.PRECISION)
-    if r is None:
-        return None
-    out, idx = r
-    return gram_solve.DeviceGram(out, gram_solve.index_tensor(idx, data.device), len(idx))
-
-
-LocalMatrix.gram_device = _local_gram_device
 
 
 def as_matrix(inputs, virtual: Optional[VirtualRows] = None) -> UpdateMatrix:

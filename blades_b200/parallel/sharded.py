@@ -24,10 +24,10 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from ..ops import attack as k_attack
-from ..ops import combine as k_combine
+from ..ops import _gram_impl
+from ..ops import gram as k_gram
 from ..ops import select as k_select
-from .matrix import UpdateMatrix, VirtualRows, resolve_scaled_rows
+from .matrix import UpdateMatrix, VirtualRows
 
 __all__ = ["ShardedMatrix"]
 
@@ -71,7 +71,8 @@ def push_plan(me: int, row0, n_local: int, ld: int, recv_ld: int, shards, recv_c
 
 
 class ShardedMatrix(UpdateMatrix):
-    def __init__(self, symm, virtual: Optional[VirtualRows] = None):
+    def __init__(self, symm, virtual: Optional[VirtualRows] = None, window=None, chunk: int = 0,
+                 last_chunk: bool = True, recv_col: int = 0):
         self.symm = symm
         self.n_rows = symm.n_total
         self.n_cols = symm.d
@@ -80,21 +81,11 @@ class ShardedMatrix(UpdateMatrix):
         self.server_step = None          # (lr,) -> theta += lr*agg fused into the final primitive
         self.step_applied = False
         self._synced = False
-        self.recv_col = 0                # column of this window inside the recv rows (pipelined aggregation)
+        self.window, self.chunk, self.last_chunk = window, chunk, last_chunk
+        self.recv_col = recv_col         # column of this window inside the recv rows (pipelined aggregation)
         self.push = _push_enabled(symm.world.size) and symm.world.size > 1 and symm.recv_ld > 0
 
     # ------------------------------------------------------------------ helpers
-    def _cols(self):
-        """This rank's coordinate range: its shard of the whole vector, or -- pipelined aggregation -- its shard of the
-        window this matrix object covers (every window is split evenly over the ranks)."""
-        if self.window is None:
-            return self.symm.my_cols
-        from ..comm.symm import coordinate_shards
-        lo, hi = int(self.window[0]), int(self.window[1])
-        c0, c1 = coordinate_shards(hi - lo, self.symm.world.size)[self.symm.world.rank]
-        return lo + c0, lo + c1
-
-    # -- push mode: rows travel by copy-engine DMA, kernels read local memory ---------------------------------------
     def _shards(self):
         """Coordinate range of every rank for this matrix object (its window, or the whole vector)."""
         from ..comm.symm import coordinate_shards
@@ -103,6 +94,12 @@ class ShardedMatrix(UpdateMatrix):
         lo, hi = int(self.window[0]), int(self.window[1])
         return [(lo + a, lo + b) for a, b in coordinate_shards(hi - lo, self.symm.world.size)]
 
+    def _cols(self):
+        """This rank's coordinate range: its shard of the whole vector, or -- pipelined aggregation -- its shard of the
+        window this matrix object covers (every window is split evenly over the ranks)."""
+        return self._shards()[self.symm.world.rank]
+
+    # -- push mode: rows travel by copy-engine DMA, kernels read local memory ---------------------------------------
     def _push_rows(self) -> None:
         """DMA this rank's rows' slice of every OTHER rank's coordinate range into that rank's ``recv`` rows
         (cudaMemcpy2DAsync over the NVLink mapping: copy engines, no SM time).  Rows replaced by virtual attack rows are
@@ -158,143 +155,49 @@ class ShardedMatrix(UpdateMatrix):
             self._barrier()
             self._synced = True
 
-    def _epilogue(self, final: bool):
+    def _rows_written(self):
+        self._barrier()
+
+    def _epilogue(self):
         s = self.symm
-        if final and self.server_step is not None:
+        if self.server_step is not None:
             self.step_applied = True
             return k_select.make_epilogue(s.agg_ptrs(), s.theta_ptrs(), s.theta.data_ptr(), float(self.server_step[0]),
-                                          mc_out=s.mc_agg_ptr(), mc_theta=s.mc_theta_ptr())
-        return k_select.make_epilogue(s.agg_ptrs(), mc_out=s.mc_agg_ptr())
+                                          mc_out=s.mc_agg_ptr(), mc_theta=s.mc_theta_ptr()), s.agg
+        return k_select.make_epilogue(s.agg_ptrs(), mc_out=s.mc_agg_ptr()), s.agg
 
-    def _finish(self) -> torch.Tensor:
+    def _finish(self):
         if self.window is None or self.last_chunk:
             self.symm.barrier()          # every shard of agg/theta has landed everywhere
-        return self.symm.agg
-
-    def gram_block_rows(self) -> list:
-        from ..ops import _gram_impl
-        return [b[2] for (ptr, ld, rows) in self.symm.block_descs() for b in _gram_impl.split_blocks(ptr, ld, rows)]
 
     def deviation_row(self, honest, dev_type: str) -> torch.Tensor:
         """q over this rank's coordinates only (the Gram pass of this rank reads no others); the rows are pulled from
         their owners, as the select kernels do."""
         self.push = False                # the Gram pass that follows pulls the rows of U itself
-        self._pre()
-        q = torch.zeros(self.n_cols, device=self.device, dtype=torch.float32)
-        c0, c1 = self._cols()
-        k_attack.deviation(self._ptrs(honest), dev_type, c0, c1, q, self.device)
-        return q
+        return super().deviation_row(honest, dev_type)
 
-    def materialize_virtual(self):
-        v = self.virtual
-        if v is not None and v.count:
-            resolve_scaled_rows(self)
-            v = self.virtual
-            self._pre()
-            s = self.symm
-            byz = set(v.byzantine)
-            honest = [i for i in range(self.n_rows) if i not in byz]
-            c0, c1 = self._cols()
-            k_attack.attack_rows(self._ptrs(honest), self._ptrs(list(v.replaced)), v.kind, v.param, c0, c1,
-                                 self.device, param_ptr=v.param_ptr())
-            self.virtual = None
-            self._barrier()
+    # ------------------------------------------------------------------ Gram
+    def _gram_blocks(self) -> list:
+        return self.symm.block_descs()
 
-    # ------------------------------------------------------------------ primitives
-    def _select(self, mode: int, b: int) -> torch.Tensor:
-        resolve_scaled_rows(self)
-        self._pre()
-        s = self.symm
-        c0, c1 = self._cols()
-        v = self.virtual
-        if v is not None and v.count:
-            byz, rep = set(v.byzantine), set(v.replaced)
-            stat = self._ptrs([i for i in range(self.n_rows) if i not in byz])
-            other = self._ptrs([i for i in range(self.n_rows) if i in byz and i not in rep])
-            k_select.launch_select(stat, other, v.count, v.kind, v.param, mode, b, c0, c1,
-                                   self._epilogue(True), self.device, param_ptr=v.param_ptr())
-        else:
-            k_select.launch_select(self._ptrs(range(self.n_rows)), [], 0, None, 0.0, mode, b, c0, c1,
-                                   self._epilogue(True), self.device)
-        return self._finish()
-
-    def trimmed_mean(self, b: int) -> torch.Tensor:
-        if self.n_rows - 2 * b <= 0:
-            raise ValueError(f"trim {b} too large for {self.n_rows} rows")
-        return self._select(0, b)
-
-    def median(self) -> torch.Tensor:
-        return self._select(1, 0)
-
-    def combine(self, weights, extra: Optional[torch.Tensor] = None, extra_weight: float = 0.0) -> torch.Tensor:
-        self.materialize_virtual()
-        self._pre()
-        s = self.symm
-        if torch.is_tensor(weights) and weights.is_cuda:
-            # device-resident weights (on-device Gram solvers): no host copy; with ``extra`` the last weight is its
-            rows = self._ptrs(range(self.n_rows))
-            if extra is not None:
-                self._keep = extra.to(self.device, torch.float32).contiguous()
-                rows = rows + [self._keep.data_ptr()]
-            c0, c1 = self._cols()
-            k_combine.launch_combine(rows, weights.to(torch.float32).contiguous(), c0, c1, self._epilogue(True), self.device)
-            return self._finish()
-        w = [float(x) for x in (weights.tolist() if hasattr(weights, "tolist") else weights)]
-        rows = self._ptrs(range(self.n_rows))
-        if extra is not None and extra_weight != 0.0:
-            rows = rows + [extra.contiguous().data_ptr()]
-            w = w + [float(extra_weight)]
-        c0, c1 = self._cols()
-        k_combine.launch_combine(rows, w, c0, c1, self._epilogue(True), self.device)
-        return self._finish()
-
-    def gram(self, extra: Optional[torch.Tensor] = None) -> np.ndarray:
-        out, idx = self._gram_scratch(extra)
-        idx_t = torch.tensor(idx, device=self.device)
-        G = out[idx_t][:, idx_t]
-        return (0.5 * (G + G.T)).double().cpu().numpy()
-
-    def gram_device(self, extra: Optional[torch.Tensor] = None):
-        from ..ops import gram_solve
-        if not gram_solve.enabled():
-            return None
-        out, idx = self._gram_scratch(extra)
-        return gram_solve.DeviceGram(out, gram_solve.index_tensor(idx, self.device), len(idx))
-
-    def _gram_scratch(self, extra: Optional[torch.Tensor] = None):
+    def _gram_pass(self, extra: Optional[torch.Tensor]):
         """Summed Gram accumulators in every rank's symmetric scratch region + the logical -> padded row list."""
-        from ..ops import _gram_impl, gram as k_gram
         self.push = False                # the Gram pass pulls the rows of U itself by TMA (peer descriptors)
         self.materialize_virtual()
         self._pre()
         s = self.symm
-        blocks = []
-        for (ptr, ld, rows) in s.block_descs():
-            blocks += _gram_impl.split_blocks(ptr, ld, rows)
-        e = 0
-        if extra is not None:
-            extra = extra.reshape(-1, self.n_cols)
-            e = extra.shape[0]
-            buf = torch.zeros(e, s.ld, device=self.device, dtype=torch.float32)
-            buf[:, : self.n_cols] = extra
-            blocks += _gram_impl.split_blocks(buf.data_ptr(), s.ld, e)
-        total_pad = sum((b[2] + 7) // 8 * 8 for b in blocks)
-        assert total_pad <= 512 and len(blocks) <= 9, "too many rows/blocks for one Gram pass"
-        tile_rows = (total_pad + 127) // 128 * 128
-        ldg = (total_pad + 31) // 32 * 32
-        # partials accumulate in this rank's replica of the symmetric scratch region; the cross-GPU sum happens in the
-        # NVSwitch (multimem.ld_reduce / multimem.st, csrc/cuda/nvls.cu) -- no NCCL call on the aggregation path
-        out = s.scratch[: tile_rows * ldg].view(tile_rows, ldg)
-        out.zero_()
         c0, c1 = s.my_cols
-        starts = _gram_impl.launch_gram(blocks, self.n_cols, c0, c1, out, k_gram.PRECISION == "tf32x3", self.device)
-        if starts is None:               # 3xTF32 staging does not fit for this row count: plain tf32
-            starts = _gram_impl.launch_gram(blocks, self.n_cols, c0, c1, out, False, self.device)
-        s.reduce_scratch(tile_rows * ldg)
-        idx = []
-        for (_, _, rows), st in zip(blocks, starts):
-            idx += list(range(st, st + rows))
-        return out, idx
+        # partials accumulate in this rank's replica of the symmetric scratch region; the cross-GPU sum happens in the
+        # NVSwitch (multimem.ld_reduce / multimem.st, csrc/cuda/nvls.cu) -- no NCCL call on the aggregation path.
+        # When the 3xTF32 staging does not fit for this row count the pass runs in plain tf32
+        r = _gram_impl.gram_pass(self._gram_blocks(), self.n_cols, c0, c1, self.device, extra,
+                                 k_gram.PRECISION == "tf32x3", tf32_fallback=True, scratch=s.scratch)
+        assert r is not None, "too many rows/blocks for one Gram pass"
+        s.reduce_scratch(r[0].numel())
+        return r
+
+    def gram(self, extra: Optional[torch.Tensor] = None) -> np.ndarray:
+        return _gram_impl.symmetrised(*self._gram_pass(extra)).double().cpu().numpy()
 
     def rows(self) -> torch.Tensor:
         self.push = False                # the gathered matrix must see materialised virtual rows in U itself

@@ -255,12 +255,9 @@ class Simulator(object):
             return agg(eng.make_matrix(None))
         if isinstance(agg, _BaseAggregator):
             from .aggregators.fltrust import Fltrust
-            matrix = eng.make_matrix(virtual)
-            if window is not None:
-                matrix.window, matrix.chunk, matrix.last_chunk, matrix.out_buffer = window, chunk, last, out
-                matrix.recv_col = recv_col
+            matrix = eng.make_matrix(virtual, window, chunk, last, out, recv_col)
             if self._opts["fuse_server_step"] and getattr(agg, "fusable_final", False) \
-                    and self.server._flat_fast_path_ok() and getattr(matrix, "use_kernels", True):
+                    and self.server._flat_fast_path_ok() and matrix.use_kernels:
                 matrix.server_step = (self.server.current_lr(),)
             self._last_matrix = matrix
             if isinstance(agg, Fltrust):
